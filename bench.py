@@ -2,6 +2,7 @@
 """Headline benchmark: V-JEPA pre-training step, clips/sec, ViT-L/16 16x224x224 synthetic, B=32 per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config vitl16|vith16|vith16_384|tiny]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is everything inside the reference's train_step() (app/vjepa/train.py:414-498) minus the three
@@ -11,6 +12,7 @@ all-reduce.  `value` times K such steps with inputs resident in HBM (CUDA events
 repeats them through the public module API with HOST inputs: pinned clips + masks copied to the device and
 the loss read back every step.  `--impl reference` times the UNMODIFIED reference's CPU path (baseline/_ref, its own
 app.vjepa.train.main, fp32) on the host cores; if baseline/_ref is absent it falls back to the CPU oracle port.
+`--dump-outputs DIR` writes what the last timed step computed to DIR (see dump_outputs).
 Prints ONE JSON line on rank 0.
 """
 import argparse
@@ -167,15 +169,18 @@ def build_training_state(cfg_name, device, world, rank):
                 scheduler=scheduler, wd_scheduler=wd_scheduler, momentum=momentum)
 
 
-def train_step(st, clips, masks_enc, masks_pred, loggers=False):
+def train_step(st, clips, masks_enc, masks_pred, loggers=False, outputs=None):
     """train_step() of app/vjepa/train.py:414-498; returns the loss (device scalar).  loggers=False is SURVEY 8d's (A)
-    math step (grad_logger x2 / adamw_logger off on both arms), loggers=True the as-shipped step (B)."""
+    math step (grad_logger x2 / adamw_logger off on both arms), loggers=True the as-shipped step (B).  A dict passed as
+    `outputs` receives the step's predictions z and targets h."""
     from jepa_b200 import step as vj
     st["scheduler"].step()
     st["wd_scheduler"].step()
     h = vj.forward_target(st["target"], clips, masks_pred)
     z = st["encoder"](clips, masks_enc)
     z = st["predictor"](z, h, masks_enc, masks_pred)
+    if outputs is not None:
+        outputs.update(z=[t.detach() for t in z], h=h)
     loss = vj.jepa_loss(z, h)
     vj.reg_loss(z)
     scaler, opt = st["scaler"], st["optimizer"]
@@ -252,6 +257,40 @@ def ncu_gemm_traffic(cfg_name):
     return None
 
 
+DUMP_SAMPLES = 1 << 20          # elements kept of each larger predicted / target array
+DUMP_PARAM_SAMPLES = 4096       # elements kept of each larger parameter tensor
+
+
+def dump_outputs(out_dir, st, loss, step_out):
+    """`--dump-outputs DIR`: what the last timed step computed, as float32 DIR/<name>.npy - loss, the predictions z_<i>
+    and targets h_<i> of every mask, and the encoder / predictor / target_encoder parameters the step left behind
+    (AdamW and EMA applied; each tensor's sample concatenated in named_parameters order).  A larger array is written as
+    its elements at positions drawn from a fixed seed, the same in every run of the same config, so the outputs of two
+    builds can be compared element for element.  About 23 MB for ViT-L/16.  The step is not bit-reproducible (split-K
+    weight gradients are reduce-adds in varying order): two runs of one build, vitl16 --steps 10 on a B200 at 1000 W,
+    differed by rel-L2 ~1e-6 in loss, ~1e-5 in the weights, 3e-3 in z and 1e-2 in h."""
+    import numpy as np
+    from jepa_b200.step import unwrap
+
+    def sample(t, n, seed):
+        flat = t.detach().reshape(-1)
+        if flat.numel() > n:
+            idx = torch.randint(flat.numel(), (n,), generator=torch.Generator().manual_seed(seed))
+            flat = flat[idx.to(flat.device)]
+        return flat.float().cpu().numpy()
+
+    arrays = {"loss": loss.detach().float().reshape(1).cpu().numpy()}
+    for i, (z, h) in enumerate(zip(step_out["z"], step_out["h"])):
+        arrays[f"z_{i}"] = sample(z, DUMP_SAMPLES, seed=2 * i)
+        arrays[f"h_{i}"] = sample(h, DUMP_SAMPLES, seed=2 * i + 1)
+    for name, key in (("encoder", "encoder"), ("predictor", "predictor"), ("target_encoder", "target")):
+        params = [p for _, p in unwrap(st[key]).named_parameters()]
+        arrays[name] = np.concatenate([sample(p, DUMP_PARAM_SAMPLES, seed=j) for j, p in enumerate(params)])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch.distributed as dist
     from jepa_b200 import _lib
@@ -314,10 +353,11 @@ def run_ours(args):
     sampler = ClockSampler(local_rank) if rank == 0 else None
     launches0 = lib.vj_launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    last = {}
     e0.record()
     t_host0 = time.perf_counter()
-    for _ in range(args.steps):
-        loss = train_step(st, clips, *step_masks(), loggers=args.loggers)
+    for i in range(args.steps):
+        loss = train_step(st, clips, *step_masks(), loggers=args.loggers, outputs=last if i == args.steps - 1 else None)
     host_enqueue_ms = (time.perf_counter() - t_host0) * 1e3 / args.steps   # host time to ENQUEUE a step (no sync inside)
     e1.record()
     sync_all()
@@ -325,6 +365,9 @@ def run_ours(args):
     launches = lib.vj_launch_count() - launches0
     clocks = sampler.stop() if sampler else None
     last_loss = float(loss)
+    if args.dump_outputs and rank == 0:   # before the passes below move the weights on
+        dump_outputs(args.dump_outputs, st, loss, last)
+    del last
     if world > 1:
         t = torch.tensor([ms_total], device=device)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -653,7 +696,13 @@ def main():
     ap.add_argument("--dynamic-masks", action="store_true", help="new collator call every step (SURVEY 8d second run)")
     ap.add_argument("--loggers", action="store_true", help="as-shipped step: grad_logger x2 + adamw_logger inside the step")
     ap.add_argument("--profile", action="store_true", help="bare steps only (for ncu); never a bench value")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, seeded samples of large arrays)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         args.steps = args.steps if args.steps is not None else 3
         args.warmup = args.warmup if args.warmup is not None else 1

@@ -41,3 +41,12 @@ def synth_state(shapes, seed, keep=()):
 
 def synth_clips(B, T, H, W, seed=0):
     return torch.randn(B, 3, T, H, W, generator=torch.Generator().manual_seed(seed))
+
+
+def sample_index(numel, n):
+    """At most n flat indices spread over a tensor of numel elements (golden-ratio sequence: no RNG, identical on
+    every machine and torch version); every index when numel <= n.  Fixtures store values at these positions only."""
+    if numel <= n:
+        return torch.arange(numel)
+    j = torch.arange(n, dtype=torch.float64)
+    return (torch.remainder(j * 0.6180339887498949, 1.0) * numel).long()

@@ -39,7 +39,13 @@ def _worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-def test_two_rank_gloo_collectives():
+def _hide_gpus(monkeypatch):
+    """The workers inherit this environment: without a visible GPU init_distributed() takes gloo, as on a CPU host."""
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
+
+
+def test_two_rank_gloo_collectives(monkeypatch):
+    _hide_gpus(monkeypatch)
     world, port = 2, _free_port()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
@@ -115,7 +121,8 @@ def _sync_worker(rank, world, port, q):
     dist.destroy_process_group()
 
 
-def test_flat_grad_sync_two_ranks():
+def test_flat_grad_sync_two_ranks(monkeypatch):
+    _hide_gpus(monkeypatch)
     world, port = 2, _free_port()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()

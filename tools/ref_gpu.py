@@ -8,14 +8,11 @@ tools/install_reference.sh) on cuda:0.  Measurement / test infrastructure only -
           `gpu-time(ms)` (src/utils/logging.py:14-31, app/vjepa/train.py:499).  This is the GPU bar SURVEY 8d asks
           for: "the same reference code on the same B200".  --loggers off stubs grad_logger / adamw_logger
           (the ~1000 host syncs per step, SURVEY 8d (A)); --loggers on is the as-shipped step (B).
-  step  : one forward/backward of the reference modules on seeded weights / clips / masks (tests/golden/common.py)
-          at a chosen width/depth, in bf16 autocast AND in fp32, dumped to a .pt file for tests/test_gpu_reference.py.
 
 The repo root holds drop-in `src/` and `app/` packages with the reference's names, so this script must run in its own
 process with the repo root OFF sys.path.
 """
 import argparse
-import copy
 import json
 import os
 import sys
@@ -30,7 +27,6 @@ if not os.path.isdir(os.path.join(REF, "app")):
     print(json.dumps({"impl": "reference-gpu", "unavailable": "baseline/_ref missing: run tools/install_reference.sh"}))
     sys.exit(0)
 sys.path.insert(0, REF)
-sys.path.insert(1, os.path.join(ROOT, "tests", "golden"))
 
 import torch  # noqa: E402
 
@@ -155,69 +151,6 @@ def run_bench(a):
     dist.destroy_process_group()
 
 
-def run_step(a):
-    """One reference step on seeded inputs (weights / clips exactly as tests/parity_util.py builds them)."""
-    from functools import partial
-    import torch.nn as nn
-    import torch.nn.functional as F
-    from common import VITL16_MASKS as MASKS, synth_clips, synth_state
-    import src.models.vision_transformer as ref_vit
-    import src.models.predictor as ref_pred
-    from src.masks.multiblock3d import MaskCollator
-    from src.masks.utils import apply_masks
-    from src.models.utils.multimask import MultiMaskWrapper, PredictorMultiMaskWrapper
-    torch.backends.cuda.matmul.allow_tf32 = False
-    torch.backends.cudnn.allow_tf32 = False
-    dev = torch.device(a.device)
-    enc = ref_vit.VisionTransformer(img_size=a.crop, patch_size=16, num_frames=a.frames, tubelet_size=2, embed_dim=a.embed_dim,
-                                    depth=a.depth, num_heads=a.heads, mlp_ratio=4, qkv_bias=True,
-                                    norm_layer=partial(nn.LayerNorm, eps=1e-6), uniform_power=True, use_sdpa=True)
-    pred = ref_pred.vit_predictor(img_size=a.crop, use_mask_tokens=True, patch_size=16, num_frames=a.frames, tubelet_size=2,
-                                  embed_dim=a.embed_dim, predictor_embed_dim=384, depth=a.pred_depth, num_heads=a.heads,
-                                  uniform_power=True, num_mask_tokens=2, zero_init_mask_tokens=True, use_sdpa=True)
-    enc_shapes = {k: tuple(v.shape) for k, v in enc.state_dict().items()}
-    pred_shapes = {k: tuple(v.shape) for k, v in pred.state_dict().items()}
-    enc.load_state_dict(synth_state(enc_shapes, seed=11, keep=("pos_embed",)), strict=False)
-    pred.load_state_dict(synth_state(pred_shapes, seed=12, keep=("pos_embed",)), strict=False)
-    tgt = copy.deepcopy(enc)
-    tgt.load_state_dict(synth_state(enc_shapes, seed=13, keep=("pos_embed",)), strict=False)
-    enc, pred, tgt = MultiMaskWrapper(enc).to(dev), PredictorMultiMaskWrapper(pred).to(dev), MultiMaskWrapper(tgt).to(dev)
-    for p in tgt.parameters():
-        p.requires_grad = False
-    clips = synth_clips(a.batch, a.frames, a.crop, a.crop, seed=0).to(dev)
-    torch.manual_seed(0)
-    coll = MaskCollator(cfgs_mask=MASKS, crop_size=a.crop, num_frames=a.frames, patch_size=16, tubelet_size=2)
-    _, me, mp = coll([torch.zeros(1) for _ in range(a.mask_batch)])
-    me, mp = [m[:a.batch].to(dev) for m in me], [m[:a.batch].to(dev) for m in mp]
-    result = {"masks_enc": [m.cpu() for m in me], "masks_pred": [m.cpu() for m in mp]}
-    for tag, dtype, mixed in (("bf16", torch.bfloat16, True), ("fp32", torch.float32, False)):
-        for net in (enc, pred):
-            for p in net.parameters():
-                p.grad = None
-        with torch.autocast(dev.type, dtype=dtype, enabled=mixed):     # train.py:453
-            with torch.no_grad():
-                h = tgt(clips)
-                h = F.layer_norm(h, (h.size(-1),))
-                h = apply_masks(h, mp, concat=False)
-            z_enc = enc(clips, me)
-            z = pred(z_enc, h, me, mp)
-            loss = sum(torch.mean(torch.abs(zi - hi)) for zi, hi in zip(z, h)) / len(mp)
-            pstd = sum(torch.sqrt(zi.var(dim=1) + 0.0001) for zi in z) / len(z)
-            loss_reg = torch.mean(F.relu(1. - pstd))
-        (loss * (65536.0 if mixed else 1.0)).backward()              # GradScaler's initial scale, unscaled below
-        inv = 1.0 / 65536.0 if mixed else 1.0
-        result[tag] = dict(
-            loss_jepa=float(loss), loss_reg=float(loss_reg),
-            h=[t.detach().float().cpu() for t in h], z=[t.detach().float().cpu() for t in z],
-            z_enc=[t.detach().float().cpu() for t in z_enc],
-            z_dtype=str(z[0].dtype), z_enc_dtype=str(z_enc[0].dtype), h_dtype=str(h[0].dtype),
-            enc_grad={n: (p.grad.detach().float() * inv).cpu() for n, p in enc.backbone.named_parameters() if p.grad is not None},
-            pred_grad={n: (p.grad.detach().float() * inv).cpu() for n, p in pred.backbone.named_parameters() if p.grad is not None})
-    torch.save(result, a.out)
-    print(json.dumps({"impl": "reference-gpu", "mode": "step", "out": a.out,
-                      "loss_bf16": result["bf16"]["loss_jepa"], "loss_fp32": result["fp32"]["loss_jepa"]}), flush=True)
-
-
 def main():
     ap = argparse.ArgumentParser()
     sub = ap.add_subparsers(dest="mode", required=True)
@@ -231,22 +164,11 @@ def main():
     b.add_argument("--out", default="")
     b.add_argument("--backend", default="nccl", help="nccl: cuda:0;  gloo: the reference's CPU path (fp32) on the host cores")
     b.add_argument("--threads", type=int, default=0)
-    s = sub.add_parser("step")
-    s.add_argument("--embed-dim", type=int, required=True)
-    s.add_argument("--heads", type=int, required=True)
-    s.add_argument("--depth", type=int, required=True)
-    s.add_argument("--pred-depth", type=int, required=True)
-    s.add_argument("--frames", type=int, default=16)
-    s.add_argument("--crop", type=int, default=224)
-    s.add_argument("--batch", type=int, default=1)
-    s.add_argument("--mask-batch", type=int, default=32)
-    s.add_argument("--out", required=True)
-    s.add_argument("--device", default="cuda:0", help="cpu only for dry runs of this script")
     a = ap.parse_args()
-    if not torch.cuda.is_available() and getattr(a, "device", "cuda:0") != "cpu" and getattr(a, "backend", "nccl") != "gloo":
+    if not torch.cuda.is_available() and a.backend != "gloo":
         print(json.dumps({"impl": "reference-gpu", "unavailable": "no CUDA device"}))
         return
-    (run_bench if a.mode == "bench" else run_step)(a)
+    run_bench(a)
 
 
 if __name__ == "__main__":
